@@ -2,6 +2,7 @@
 """bench.py -- BASELINE.json's headline metric: Mrays/s, primary + 1-bounce AO rays.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scaling strong|weak]
+                    [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1]): procedural 100,002-triangle sphere grid, 1920x1080, 16 spp of jittered
 pinhole primary rays + one cosine-hemisphere AO ray per primary hit (closest-hit queries, as the reference's
@@ -28,6 +29,10 @@ CheckForOccluder does).  One "step" = one pass over all samples of the image.
   --impl reference : the UNMODIFIED reference (oracle/_ref, built from /root/reference/nanort.h) -- or the oracle port
             when that is absent -- traces a bounded sample of the very same ray arrays on the host cores, after a
             thread sweep {1, 2, 4, ..., nproc}; rank 0 only.
+  --dump-outputs DIR : after the timed steps, what the last timed step computed, as DIR/<name>.npy (float32 / float64):
+            frame.npy, the HEIGHT x WIDTH framebuffer (per pixel, the number of samples whose AO ray was not occluded;
+            primary misses count as unoccluded).  The inputs depend on the arguments only, so two builds can be
+            compared output for output.  (--impl reference traces a sample sized by a timing calibration: no dump.)
 """
 from __future__ import annotations
 
@@ -147,6 +152,12 @@ def config_dict(n_gpus, scaling, spp_total):
                      "16 Mi-ray wave = 2.6 x the 126 MB L2; scene + BVH (10 MB) stay cache-resident by design",
         "parallelism": f"ray-tile sharding x{n_gpus}",
     }
+
+
+def dump_outputs(out_dir, **arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, np.float32 if a.dtype.itemsize <= 4 else np.float64))
 
 
 # ----------------------------------------------------------------------------------- reference arm
@@ -672,7 +683,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the additional BASELINE configs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 0)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -780,6 +796,8 @@ def main():
     sync_all()
     t_end = time.time()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, frame=(frame if distributed else accum).view(HEIGHT, WIDTH).cpu().numpy())
     # the same steps again for >= 2 s (not part of `value`): clocks and thermals are sampled over a region long enough
     # for nvidia-smi's 50 ms period to see them; its rate is reported as `sustained`
     e2, e3 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)

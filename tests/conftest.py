@@ -18,13 +18,3 @@ def port():
 
     orc.make()
     return orc.Port()
-
-
-@pytest.fixture(scope="session")
-def reference():
-    """The unmodified reference behind oracle/_ref (prebuilt in the authoring container)."""
-    from oracle import orc
-
-    if not orc.Reference.available(True):
-        pytest.skip("oracle/_ref not built (no /root/reference in this environment)")
-    return orc.Reference(True)

@@ -1,5 +1,50 @@
 """Shared parity checker: GPU results vs the oracle, with exact-t tie classification (SURVEY.md F3)."""
+import hashlib
+import json
+import os
+
 import numpy as np
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+REF_DIFF = ("differs from the unmodified reference's recorded result; with oracle/_ref built, "
+            "tests/golden/make_reference_golden.py reruns the reference on the same inputs for a per-ray comparison")
+
+
+def digest(*arrays):
+    """SHA-256 over the dtype, shape and raw bytes of the arrays: a bit-for-bit fingerprint of a result of the
+    unmodified reference that is too large to store (tests/golden/reference_digests.json)."""
+    h = hashlib.sha256()
+    for a in arrays:
+        a = np.ascontiguousarray(a)
+        h.update(f"{a.dtype.str}{a.shape}".encode())
+        h.update(a.tobytes())
+    return h.hexdigest()
+
+
+def tree_digest(nodes, indices):
+    """Node array + indices_.  A leaf's `axis` is never written by the reference (nanort.h:1795-1813): zeroed."""
+    nodes = np.array(nodes, copy=True)
+    nodes["axis"][nodes["flag"] != 0] = 0
+    return digest(nodes, np.asarray(indices, np.uint32))
+
+
+def hits_digest(hits, mask):
+    """Hit flags of every ray + every field (padding aside) of the records of the rays that hit."""
+    mask = np.asarray(mask, np.uint8)
+    hit = mask == 1
+    return digest(mask, *(hits[k][hit] for k in hits.dtype.names if k != "pad"))
+
+
+def list_digest(lists):
+    """Node-hit lists, one (t_min, t_max, node_id) triple of arrays per ray."""
+    return digest(*(x for tmin, tmax, ids in lists for x in (np.array([len(ids)], np.int64), tmin, tmax, ids)))
+
+
+def reference_golden():
+    with open(os.path.join(GOLDEN, "reference_digests.json")) as f:
+        return json.load(f)
 
 
 def compare_hits(port, verts, faces, rays, got_hits, got_mask, want_hits, want_mask, topts=None, cpp11=True,

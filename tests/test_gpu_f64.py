@@ -1,9 +1,12 @@
 """BVHAccel<double> on the GPU (nrt_build_f64 / nrt_traverse_f64).  Checker: the unmodified reference's fp64
-instantiation (oracle/_ref, ref64_*) and the committed golden vectors of the reference's regression program."""
+instantiation, through its results recorded in tests/golden (fingerprints in reference_digests.json, the reference's
+regression program in regression30.npz) and through the oracle's double restatement pinned to them."""
 import os
 
 import numpy as np
 import pytest
+
+from helpers import REF_DIFF, hits_digest, reference_golden, tree_digest
 
 pytestmark = pytest.mark.gpu
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -90,19 +93,18 @@ def test_f64_hits_match_the_reference(cpp11):
     from nanort_b200 import api
     from oracle import orc
 
-    if not orc.Reference.available(cpp11):
-        pytest.skip("oracle/_ref not built")
-    ref = orc.ReferenceF64(cpp11)
-    assert ref.sizes() == [64, 72, 32, 32, 16]
+    port = orc.Port64()
     v64, f = _scene64()
     rays = _rays64(v64, 60000, seed=4)
     acc = api.BVHAccelF64()
     acc.Build(len(f), v64, f)
     flags = api.TRAVERSE_CONFORMANCE | (0 if cpp11 else api.TRAVERSE_CPP03_INVERSE)
     gh, gm = acc.Traverse(rays, flags=flags)
-    # (1) the reference's own Build + Traverse in double: same hits; same bits for the same primitive
-    racc = ref.build(v64, f)
-    rh, rm = racc.traverse(rays, threads=8)
+    # (1) the reference's own Build + Traverse in double (the restatement's, checked against the reference's recorded
+    # result): same hits; same bits for the same primitive
+    rn, ri, _ = port.build(v64, f, None, orc.MODE_CPP11 if cpp11 else 0)
+    rh, rm = port.traverse(rn, ri, v64, f, rays, cpp11=cpp11, threads=8)
+    assert hits_digest(rh, rm) == reference_golden()[f"gpu_f64_hits/{cpp11}"], REF_DIFF
     assert rm.sum() > 5000 and np.array_equal(rm, gm)
     hit = rm == 1
     same = hit & (rh["prim_id"] == gh["prim_id"])
@@ -110,16 +112,16 @@ def test_f64_hits_match_the_reference(cpp11):
         assert np.array_equal(rh[k][same].view(np.uint64), gh[k][same].view(np.uint64)), k
     other = hit & ~same  # a different primitive only at exactly the same distance (shared edges)
     assert other.sum() <= 0.002 * hit.sum() and np.array_equal(rh["t"][other], gh["t"][other])
-    # (2) the reference walking the GPU's node array (its own Load): everything bit-equal, ties included
-    adopted = ref.adopt(acc.GetNodes(), acc.GetIndices(), v64, f)
-    ah, am = adopted.traverse(rays, threads=8)
+    # (2) the reference's Traverse walking the GPU's node array: everything bit-equal, ties included
+    gn, gi = acc.GetNodes(), acc.GetIndices()
+    ah, am = port.traverse(gn, gi, v64, f, rays, cpp11=cpp11, threads=8)
     assert np.array_equal(am, gm)
     for k in ("t", "u", "v", "prim_id"):
         assert ah[k][hit].tobytes() == gh[k][hit].tobytes(), k
     # (3) trace options
     o = orc.trace_options(cull_back_face=1, skip_prim_id=int(gh["prim_id"][hit][0]))
     gh2, gm2 = acc.Traverse(rays[:8000], options=o, flags=flags)
-    ah2, am2 = adopted.traverse(rays[:8000], topts=o, threads=4)
+    ah2, am2 = port.traverse(gn, gi, v64, f, rays[:8000], topts=o, cpp11=cpp11, threads=4)
     assert np.array_equal(am2, gm2) and ah2[am2 == 1].tobytes() == gh2[gm2 == 1].tobytes()
     assert gm2.sum() < gm[:8000].sum()
 
@@ -127,31 +129,32 @@ def test_f64_hits_match_the_reference(cpp11):
 @pytest.mark.parametrize("cpp11", [True, False])
 def test_f64_adopted_reference_tree_is_bit_exact(cpp11):
     """BVHAccel<double>::Load path (nrt_adopt_f64): the CPU reference's own double tree walked on the GPU gives the
-    reference's records bit for bit -- hit flag, prim_id (ties included), t, u, v."""
+    reference's records bit for bit -- hit flag, prim_id (ties included), t, u, v.  The tree is the restatement's,
+    which is the reference's (tests/golden/reference_digests.json)."""
     from nanort_b200 import api
     from oracle import orc
 
-    if not orc.Reference.available(cpp11):
-        pytest.skip("oracle/_ref not built")
-    ref = orc.ReferenceF64(cpp11)
+    want = reference_golden()[f"gpu_f64_adopted/{cpp11}"]
+    port = orc.Port64()
     v64, f = _scene64(seed=9)
     rays = _rays64(v64, 40000, seed=10)
-    racc = ref.build(v64, f)
-    rh, rm = racc.traverse(rays, threads=8)
+    rn, ri, _ = port.build(v64, f, None, orc.MODE_CPP11 if cpp11 else 0)
+    assert tree_digest(rn, ri) == want["tree"], REF_DIFF
+    rh, rm = port.traverse(rn, ri, v64, f, rays, cpp11=cpp11, threads=8)
+    assert hits_digest(rh, rm) == want["hits"], REF_DIFF
     acc = api.BVHAccelF64()
-    assert acc.Adopt(racc.nodes(), racc.indices(), v64, f)
+    assert acc.Adopt(rn, ri, v64, f)
     gh, gm = acc.Traverse(rays, flags=api.TRAVERSE_CONFORMANCE | (0 if cpp11 else api.TRAVERSE_CPP03_INVERSE))
     assert rm.sum() > 3000 and np.array_equal(rm, gm)
     hit = rm == 1
     for k in ("t", "u", "v", "prim_id"):
         assert rh[k][hit].tobytes() == gh[k][hit].tobytes(), k
     a, b = acc.BoundingBox()
-    ra, rb = racc.bounding_box()
-    assert np.array_equal(a, ra) and np.array_equal(b, rb)
+    assert a.tolist() == want["bbox"][0] and b.tolist() == want["bbox"][1]
     with pytest.raises(api.NanortB200Error):  # foreign data is validated
-        bad = racc.nodes().copy()
+        bad = rn.copy()
         bad["data"][np.nonzero(bad["flag"] == 0)[0][0], 0] = len(bad) + 3
-        api.BVHAccelF64().Adopt(bad, racc.indices(), v64, f)
+        api.BVHAccelF64().Adopt(bad, ri, v64, f)
 
 
 @pytest.mark.parametrize("cpp11", [True, False])
@@ -183,11 +186,25 @@ def test_f64_against_the_c_restatement(cpp11):
         assert qh[k][qm == 1].tobytes() == ah[k][am == 1].tobytes(), k
 
 
+def conformance_cases():
+    from nanort_b200 import scenes as S
+    from oracle import orc
+
+    cases = [(_scene64(seed=21), None), (_scene64(seed=22), orc.build_options_f64(min_leaf_primitives=1, bin_size=16)),
+             (_scene64(seed=23), orc.build_options_f64(max_tree_depth=6))]
+    v, f = S.make_scene("cornell")
+    cases.append(((v.astype(np.float64) * (1.0 + 1e-13), f), None))
+    v, f = S.sphere_grid(nx=6, nz=5)  # 30,000 triangles: above min_primitives_for_parallel_build -> joined node order
+    rng = np.random.default_rng(5)
+    cases.append(((v.astype(np.float64) + 1e-10 * rng.standard_normal(v.shape), f), None))
+    return cases
+
+
 @pytest.mark.parametrize("cpp11", [True, False])
 def test_f64_conformance_build_writes_the_references_arrays(cpp11):
     """nrt_build_f64_ex(NRT_BUILD_REFERENCE_TREE): the device writes the very BVHNode<double> array and indices_ that
     BVHAccel<double>::Build writes -- checked against the oracle's double instantiation (pinned to the unmodified
-    reference's BVHAccel<double> by tests/test_oracle_f64.py) and, where oracle/_ref exists, against the reference itself:
+    reference's BVHAccel<double> by tests/test_oracle_f64.py) and against the reference's own trees (recorded fingerprints):
     every field of every node, every index, the statistics, for several scenes and option sets -- coordinates that do not
     survive a round trip through float, so a float-precision split decision would show."""
     from nanort_b200 import api, scenes as S
@@ -196,14 +213,10 @@ def test_f64_conformance_build_writes_the_references_arrays(cpp11):
     port = orc.Port64()
     mode = orc.MODE_CPP11 if cpp11 else 0
     flags = api.BUILD_REFERENCE_TREE | (0 if cpp11 else api.BUILD_REFERENCE_CPP03_ORDER)
-    cases = [(_scene64(seed=21), None), (_scene64(seed=22), orc.build_options_f64(min_leaf_primitives=1, bin_size=16)),
-             (_scene64(seed=23), orc.build_options_f64(max_tree_depth=6))]
-    v, f = S.make_scene("cornell")
-    cases.append(((v.astype(np.float64) * (1.0 + 1e-13), f), None))
-    v, f = S.sphere_grid(nx=6, nz=5)  # 30,000 triangles: above min_primitives_for_parallel_build -> joined node order
-    rng = np.random.default_rng(5)
-    cases.append(((v.astype(np.float64) + 1e-10 * rng.standard_normal(v.shape), f), None))
-    for (v64, f), opts in cases:
+    cases = conformance_cases()
+    ref_trees = reference_golden()[f"gpu_f64_conformance/{cpp11}"]
+    assert len(ref_trees) == len(cases)
+    for ((v64, f), opts), ref_tree in zip(cases, ref_trees):
         want_nodes, want_idx, _ = port.build(v64, f, opts, mode)
         acc = api.BVHAccelF64()
         assert acc.Build(len(f), v64, f, options=opts, flags=flags)
@@ -216,12 +229,7 @@ def test_f64_conformance_build_writes_the_references_arrays(cpp11):
         assert np.array_equal(nodes["axis"][br], want_nodes["axis"][br])  # the reference leaves leaf.axis uninitialised
         st = acc.GetStatistics()
         assert st["num_leaf_nodes"] == int((nodes["flag"] == 1).sum()) and st["num_branch_nodes"] == int(br.sum())
-        if orc.Reference.available(cpp11):
-            racc = orc.ReferenceF64(cpp11).build(v64, f, opts)
-            rn = racc.nodes()
-            assert np.array_equal(racc.indices(), idx)
-            for k in ("bmin", "bmax", "flag", "data"):
-                assert rn[k].tobytes() == nodes[k].tobytes(), k
+        assert tree_digest(nodes, idx) == ref_tree, REF_DIFF
         # and the conformance walk over it gives the oracle's records, ties included
         rays = _rays64(v64, 5000, seed=31)
         tf = api.TRAVERSE_CONFORMANCE | (0 if cpp11 else api.TRAVERSE_CPP03_INVERSE)

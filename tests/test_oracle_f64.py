@@ -1,23 +1,21 @@
 """CPU: the C restatement instantiated for double (oracle/liborc64.so) against the unmodified reference's
-BVHAccel<double> (oracle/_ref, ref64_*): record sizes, node array, indices_, and every hit record, bit for bit,
-in both build modes / vsafe_inverse conventions; plus the reference's regression program in its native precision."""
+BVHAccel<double>: record sizes, node array, indices_, and every hit record, bit for bit, in both build modes /
+vsafe_inverse conventions (the reference's results as fingerprints, tests/golden/reference_digests.json); plus the
+reference's regression program in its native precision."""
 import os
 
 import numpy as np
 import pytest
 
+from helpers import REF_DIFF, hits_digest, reference_golden, tree_digest
 from nanort_b200 import scenes as S
 from oracle import orc
 
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-
-
-def _cmp_nodes(a, b):
-    assert len(a) == len(b)
-    for k in ("bmin", "bmax", "flag", "data"):
-        assert a[k].tobytes() == b[k].tobytes(), k
-    br = a["flag"] == 0
-    assert np.array_equal(a["axis"][br], b["axis"][br])  # a leaf's axis is never written by the reference
+SCENES = [("cornell", {}), ("sphere_grid", dict(nx=3, nz=3)), ("terrain", dict(n=80))]
+BUILD_VARIANTS = (dict(min_leaf_primitives=1), dict(bin_size=8, min_leaf_primitives=8), dict(max_tree_depth=6),
+                  dict(shallow_depth=2, min_primitives_for_parallel_build=1000))
+TRACE_VARIANTS = (dict(cull_back_face=1), dict(skip_prim_id=17), dict(prim_ids_range=(100, 900)))
 
 
 def _scene64(name, kw, seed):
@@ -43,49 +41,35 @@ def _rays64(v64, n, seed, hostile=False):
     return r
 
 
-@pytest.mark.parametrize("name,kw", [("cornell", {}), ("sphere_grid", dict(nx=3, nz=3)), ("terrain", dict(n=80))])
+@pytest.mark.parametrize("name,kw", SCENES)
 @pytest.mark.parametrize("cpp11", [True, False])
 def test_port64_equals_reference_double(name, kw, cpp11):
-    if not orc.Reference.available(cpp11):
-        pytest.skip("oracle/_ref not built")
-    ref, port = orc.ReferenceF64(cpp11), orc.Port64()
-    assert ref.sizes() == port.sizes() == [64, 72, 32, 32, 16]
+    g = reference_golden()
+    port = orc.Port64()
+    assert g["ref64_sizes"] == port.sizes() == [64, 72, 32, 32, 16]
+    want = g[f"f64_vs_ref/{name}/{cpp11}"]
     v64, f = _scene64(name, kw, seed=2)
-    racc = ref.build(v64, f)
     nodes, idx, st = port.build(v64, f, None, orc.MODE_CPP11 if cpp11 else 0)
-    _cmp_nodes(racc.nodes(), nodes)
-    assert np.array_equal(racc.indices(), idx)
+    assert tree_digest(nodes, idx) == want["tree"], REF_DIFF
     assert st["num_leaf_nodes"] == st["num_branch_nodes"] + 1
     for hostile in (False, True):
         rays = _rays64(v64, 12000, seed=6, hostile=hostile)
-        rh, rm = racc.traverse(rays, threads=4)
         ph, pm = port.traverse(nodes, idx, v64, f, rays, cpp11=cpp11, threads=4)
-        assert np.array_equal(rm, pm)
-        for k in ("t", "u", "v", "prim_id"):
-            assert rh[k][rm == 1].tobytes() == ph[k][pm == 1].tobytes(), (k, hostile)
-    assert rm.sum() > 100
+        assert hits_digest(ph, pm) == want[f"hits/{hostile}"], (hostile, REF_DIFF)
+    assert pm.sum() > 100
 
 
 def test_port64_build_options_and_trace_options():
-    if not orc.Reference.available(True):
-        pytest.skip("oracle/_ref not built")
-    ref, port = orc.ReferenceF64(True), orc.Port64()
+    g = reference_golden()
+    port = orc.Port64()
     v64, f = _scene64("sphere_grid", dict(nx=2, nz=2), seed=4)
-    for okw in (dict(min_leaf_primitives=1), dict(bin_size=8, min_leaf_primitives=8), dict(max_tree_depth=6),
-                dict(shallow_depth=2, min_primitives_for_parallel_build=1000)):
-        o = orc.build_options_f64(**okw)
-        racc = ref.build(v64, f, o)
-        nodes, idx, _ = port.build(v64, f, o, orc.MODE_CPP11)
-        _cmp_nodes(racc.nodes(), nodes)
-        assert np.array_equal(racc.indices(), idx), okw
+    for okw in BUILD_VARIANTS:
+        nodes, idx, _ = port.build(v64, f, orc.build_options_f64(**okw), orc.MODE_CPP11)
+        assert tree_digest(nodes, idx) == g[f"f64_vs_ref_options/{sorted(okw.items())}"], (okw, REF_DIFF)
     rays = _rays64(v64, 6000, seed=8)
-    for tkw in (dict(cull_back_face=1), dict(skip_prim_id=17), dict(prim_ids_range=(100, 900))):
-        t = orc.trace_options(**tkw)
-        rh, rm = racc.traverse(rays, topts=t)
-        ph, pm = port.traverse(nodes, idx, v64, f, rays, topts=t)
-        assert np.array_equal(rm, pm) and rh[rm == 1].tobytes()[:0] == b""
-        for k in ("t", "u", "v", "prim_id"):
-            assert rh[k][rm == 1].tobytes() == ph[k][pm == 1].tobytes(), (k, tkw)
+    for tkw in TRACE_VARIANTS:  # on the tree of the last build option set
+        ph, pm = port.traverse(nodes, idx, v64, f, rays, topts=orc.trace_options(**tkw))
+        assert hits_digest(ph, pm) == g[f"f64_vs_ref_options/{sorted(tkw.items())}"], (tkw, REF_DIFF)
 
 
 def test_port64_regression30_native_precision():

@@ -1,41 +1,41 @@
-"""CPU: the oracle port against the live reference (oracle/_ref) -- bit-for-bit, both build modes."""
+"""CPU: the oracle port against the unmodified reference -- bit-for-bit, both build modes.  The reference's results are
+recorded as fingerprints in tests/golden/reference_digests.json (tests/golden/make_reference_golden.py)."""
 import numpy as np
 import pytest
 
+from helpers import REF_DIFF, hits_digest, reference_golden, tree_digest
 
-def _cmp_nodes(a, b):
-    assert len(a) == len(b)
-    for k in ("bmin", "bmax"):
-        assert np.array_equal(a[k].view(np.uint32), b[k].view(np.uint32))
-    assert np.array_equal(a["flag"], b["flag"]) and np.array_equal(a["data"], b["data"])
-    br = a["flag"] == 0
-    assert np.array_equal(a["axis"][br], b["axis"][br])
+SCENES = [("cornell", {}), ("sphere_grid", dict(nx=3, nz=3)), ("terrain", dict(n=80))]
+BUILD_VARIANTS = (dict(min_leaf_primitives=1), dict(bin_size=8), dict(max_tree_depth=6), dict(min_leaf_primitives=16))
+TRACE_VARIANTS = (dict(cull_back_face=1), dict(skip_prim_id=17), dict(prim_ids_range=(1000, 3000)))
 
 
-@pytest.mark.parametrize("name,kw", [("cornell", {}), ("sphere_grid", dict(nx=3, nz=3)), ("terrain", dict(n=80))])
+def scene_rays(name, v):
+    from nanort_b200 import scenes as S
+
+    cam = S.scene_camera(name, 128, 96)
+    return np.concatenate([S.primary_rays(cam, 128, 96, spp=1, seed=5),
+                           S.incoherent_rays(v.min(axis=0), v.max(axis=0), 30000, seed=6)])
+
+
+@pytest.mark.parametrize("name,kw", SCENES)
 @pytest.mark.parametrize("cpp11", [True, False])
 def test_port_equals_reference(port, name, kw, cpp11):
     from oracle import orc
     from nanort_b200 import scenes as S
 
-    if not orc.Reference.available(cpp11):
-        pytest.skip("oracle/_ref not built")
-    ref = orc.Reference(cpp11)
-    assert ref.sizes() == [40, 36, 16, 28, 16]
+    g = reference_golden()
+    assert g["ref_sizes"] == [40, 36, 16, 28, 16]
+    assert [d.itemsize for d in (orc.NODE_DTYPE, orc.RAY_DTYPE, orc.HIT_DTYPE, orc.BUILD_OPT_DTYPE,
+                                 orc.TRACE_OPT_DTYPE)] == g["ref_sizes"]
+    want = g[f"vs_ref/{name}/{cpp11}"]
     v, f = S.make_scene(name, **kw)
-    ra = ref.build(v, f)
     pn, pi, ps = port.build(v, f, mode=orc.MODE_CPP11 if cpp11 else 0)
-    _cmp_nodes(ra.nodes(), pn)
-    assert np.array_equal(ra.indices(), pi)
-    assert ra.stats() == ps
-    cam = S.scene_camera(name, 128, 96)
-    rays = np.concatenate([S.primary_rays(cam, 128, 96, spp=1, seed=5),
-                           S.incoherent_rays(v.min(axis=0), v.max(axis=0), 30000, seed=6)])
-    rh, rm = ra.traverse(rays, threads=4)
+    assert tree_digest(pn, pi) == want["tree"], REF_DIFF
+    assert list(ps.values()) == want["stats"]
+    rays = scene_rays(name, v)
     ph, pm, ctr = port.traverse(pn, pi, v, f, rays, cpp11=cpp11, threads=4, counters=True)
-    assert np.array_equal(rm, pm)
-    hit = rm.astype(bool)
-    assert np.array_equal(rh[hit].view(np.uint32), ph[hit].view(np.uint32))
+    assert hits_digest(ph, pm) == want["hits"], REF_DIFF
     assert ctr["nodes_popped"] >= len(rays)
 
 
@@ -44,26 +44,18 @@ def test_reference_option_variants(port):
     from oracle import orc
     from nanort_b200 import scenes as S
 
-    if not orc.Reference.available(True):
-        pytest.skip("oracle/_ref not built")
-    ref = orc.Reference(True)
+    g = reference_golden()
     v, f = S.make_scene("sphere_grid", nx=2, nz=2)
     rays = S.incoherent_rays(v.min(axis=0), v.max(axis=0), 20000, seed=8)
-    for okw in (dict(min_leaf_primitives=1), dict(bin_size=8), dict(max_tree_depth=6), dict(min_leaf_primitives=16)):
-        o = orc.build_options(**okw)
-        ra = ref.build(v, f, o)
-        pn, pi, ps = port.build(v, f, o)
-        _cmp_nodes(ra.nodes(), pn)
-        assert ra.stats() == ps
-    ra = ref.build(v, f)
+    for okw in BUILD_VARIANTS:
+        pn, pi, ps = port.build(v, f, orc.build_options(**okw))
+        want = g[f"vs_ref_options/{sorted(okw.items())}"]
+        assert tree_digest(pn, pi) == want["tree"], (okw, REF_DIFF)
+        assert list(ps.values()) == want["stats"], okw
     pn, pi, _ = port.build(v, f)
-    for tkw in (dict(cull_back_face=1), dict(skip_prim_id=17), dict(prim_ids_range=(1000, 3000))):
-        t = orc.trace_options(**tkw)
-        rh, rm = ra.traverse(rays, topts=t)
-        ph, pm = port.traverse(pn, pi, v, f, rays, topts=t)
-        assert np.array_equal(rm, pm)
-        hit = rm.astype(bool)
-        assert np.array_equal(rh[hit].view(np.uint32), ph[hit].view(np.uint32))
+    for tkw in TRACE_VARIANTS:
+        ph, pm = port.traverse(pn, pi, v, f, rays, topts=orc.trace_options(**tkw))
+        assert hits_digest(ph, pm) == g[f"vs_ref_options/{sorted(tkw.items())}"], (tkw, REF_DIFF)
 
 
 @pytest.mark.parametrize("cpp11", [True, False])
@@ -73,16 +65,10 @@ def test_port_equals_reference_on_hostile_rays_and_degenerate_triangles(port, cp
     from oracle import orc
     from edge_cases import degenerate_mesh, hostile_rays
 
-    if not orc.Reference.available(cpp11):
-        pytest.skip("oracle/_ref not built")
-    ref = orc.Reference(cpp11)
+    want = reference_golden()[f"vs_ref_hostile/{cpp11}"]
     v, f = degenerate_mesh()
-    acc = ref.build(v, f)
     nodes, idx, _ = port.build(v, f, None, orc.MODE_CPP11 if cpp11 else 0)
-    _cmp_nodes(acc.nodes(), nodes)
-    assert np.array_equal(acc.indices(), idx)
+    assert tree_digest(nodes, idx) == want["tree"], REF_DIFF
     rays = hostile_rays(v[:34 * 3].min(axis=0) - 1, v[:34 * 3].max(axis=0) + 1)
-    rh, rm = acc.traverse(rays)
     ph, pm = port.traverse(nodes, idx, v, f, rays, cpp11=cpp11)
-    assert np.array_equal(rm, pm)
-    assert rh[rm == 1].tobytes() == ph[pm == 1].tobytes()
+    assert hits_digest(ph, pm) == want["hits"], REF_DIFF
